@@ -3,6 +3,7 @@
 bench.py -- env-steps/sec of the gym-fx env.step() hot path (BASELINE.json metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2|cfg3|cfg4|cfg5]
+                  [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" = one env.step() of every env of the workload.  Default
@@ -22,6 +23,9 @@ ours:       K steps through fxenv_step_many in batches of <= 500 (actions pre-ge
             `closed_loop` = BASELINE configs[3] shape with the policy IN the loop (fused tcgen05 actor-critic kernel <->
             env step, VecFxEnv.rollout) and one PPO update with its NCCL all-reduces (time per update and share).
             `other_workloads` (N=1) = short runs of BASELINE configs[2] and configs[4] (cfg3 / cfg5 shapes).
+            --dump-outputs DIR: after the timed steps, rank 0 writes what the last timed step handed back (see
+            dump_outputs) as DIR/<name>.npy.  Inputs are seeded, so two builds run with the same arguments can be
+            compared output for output.
 reference:  the CPU arm: the oracle port (oracle/fxenv_oracle.c; the Python reference cannot travel to the GPU box)
             stepping the SAME workload with all host threads.
 """
@@ -408,6 +412,27 @@ def closed_loop_block(K, rank, world, dev, dist):
     }
 
 
+DUMP_BUDGET = 60 << 20   # array bytes of one --dump-outputs: the files, .npy headers included, stay under 64 MB
+
+
+def dump_outputs(path, env, ring, rews, terms, last):
+    """--dump-outputs: what the last timed step (index `last` of its fxenv_step_many batch) handed its caller -- every
+    env's observation row, reward and terminated flag -- and the equity of every env after it, as <path>/<name>.npy
+    (float32 / float64).  `env_index` holds the env ids of the rows; when the full arrays would exceed DUMP_BUDGET,
+    the rows are a fixed seeded sample of the envs."""
+    N = ring.shape[1]
+    out = {"obs": ring[last % ring.shape[0]], "reward": rews[last], "terminated": terms[last].float(),
+           "equity": env.info()["equity"]}
+    per_env = sum(v[0].numel() * v.element_size() for v in out.values()) + 8   # + 8: env_index
+    idx = np.arange(N)
+    if per_env * N > DUMP_BUDGET:
+        idx = np.sort(np.random.default_rng(0).choice(N, DUMP_BUDGET // per_env, replace=False))
+    os.makedirs(path, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(path, name + ".npy"), v.cpu().numpy()[idx])
+    np.save(os.path.join(path, "env_index.npy"), idx.astype(np.float64))
+
+
 def run_ours(args, rank, world, local_rank):
     import torch
     from gym_fx_b200.sharding import check_pair_alignment, shard_starts
@@ -485,6 +510,8 @@ def run_ours(args, rank, world, local_rank):
     engine = env.step_many_engine(chunk)
     overflow = int((env.info()["flags"] & 16).ne(0).sum().item())
     term_frac = float(terms.float().mean().item())
+    if args.dump_outputs and rank == 0:      # before anything below reuses the buffers or steps the envs further
+        dump_outputs(args.dump_outputs, env, ring, rews, terms, (rem or chunk) - 1)
 
     # ---- e2e: reference-facing host-buffer call, copies inside the timed region; median of 5 repeats of K steps
     Ke, reps = min(K, 400), 5
@@ -615,11 +642,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-closed-loop", action="store_true", help="skip the policy-in-the-loop (cfg4) block")
     ap.add_argument("--no-other-workloads", action="store_true", help="skip the short cfg3 / cfg5 runs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (--impl ours)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
         run_reference(args, rank, world)
         return
     if world != args.gpus and world == 1 and args.gpus > 1:
